@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the ScanFold scanning hot path on B200 (contract: see DESIGN.md "Measurement").
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload C2]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload C2] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one record shard: for every window the native MFE fold
 (+ structure), the partition function / ensemble diversity / centroid, r shuffles generated on the
@@ -16,6 +16,12 @@ of ~29.8 k windows of an N x 29,903-nt record (weak scaling).
 `--impl reference`  the reference's CPU path.  ViennaRNA is not installable here (no network, not in the
           image), so this arm times oracle/ (the CPU restatement of the same algorithms) on all host
           cores over a bounded sample of the same workload.
+`--dump-outputs DIR`  after the timed steps, write what the last step of each arm computed as DIR/<name>.npy
+          (float64, integers exact, 64 MB at most): scan_* = the ScanPlan.fetch() arrays of the device arm,
+          e2e_* = the per-nucleotide results, window columns and partner table of the end-to-end arm.  Large
+          per-window or per-entry arrays are a fixed, seeded sample (the indices are dumped beside them).  With
+          several GPUs rank 0 writes: its own shard of the device arm and partner table, the gathered rest.
+          The inputs are seeded, so two builds run with the same arguments can be compared file by file.
 """
 import argparse
 import json
@@ -260,6 +266,57 @@ def result_sha(agg, table_digest, table):
     return h.hexdigest()[:16]
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_SAMPLE_WINDOWS = 4096      # rows of the [n, r] shuffle energies and [n, W] structures
+DUMP_SAMPLE_ENTRIES = 65536     # entries of the partner table
+NT_RESULT_FIELDS = ("coord", "part", "cov_z", "mean_z", "mean_mfe", "mean_ed", "total_windows", "num_bp")
+
+
+def sample_indices(n, k, seed):
+    """sorted indices of a fixed, seeded sample of k out of n (all n when n <= k)"""
+    if n <= k:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, size=k, replace=False))
+
+
+def scan_outputs(res):
+    """ScanPlan.fetch() of the device arm: per-window columns in full, the wide arrays for a sample of windows"""
+    out = {"scan_" + k: getattr(res, k) for k in ("mfe_dcal", "native_unconstrained_dcal", "ed", "ensemble_dG")}
+    rows = sample_indices(res.n, DUMP_SAMPLE_WINDOWS, 1)
+    out["scan_sample_windows"] = rows
+    for k in ("shuffle_dcal", "pair_tbl", "centroid_tbl"):
+        out["scan_" + k] = getattr(res, k)[rows]
+    return out
+
+
+def e2e_outputs(agg, wtable, ptable):
+    """the end-to-end arm: per-nucleotide results, per-window columns, the partner table for a sample of entries"""
+    out = {"e2e_nt_" + k: getattr(agg, k) for k in NT_RESULT_FIELDS}
+    for k in ("mfe", "z", "p", "ed"):
+        out["e2e_window_" + k] = getattr(wtable, k)
+    if wtable.final is not None:
+        out["e2e_final_window_mfe_z_p_ed"] = [wtable.final[k] for k in ("mfe", "z", "p", "ed")]
+    out["e2e_partner_nt_ptr"] = ptable.nt_ptr
+    out["e2e_partner_coord"] = ptable.coord
+    entries = sample_indices(len(ptable.partner), DUMP_SAMPLE_ENTRIES, 2)
+    out["e2e_partner_sample_entries"] = entries
+    for k in ("partner", "count", "first_seen"):
+        out["e2e_partner_" + k] = getattr(ptable, k)[entries]
+    out["e2e_partner_sums"] = ptable.sums[:, entries]
+    return out
+
+
+def write_outputs(path, arrays):
+    """every array as <path>/<name>.npy in float64 (exact for the integer arrays: all below 2^53)"""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit("bench.py: --dump-outputs would write %d bytes, more than %d" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -314,6 +371,7 @@ def run_ours(args):
     barrier()
     clocks = sampler.stop()
     ms_dev = ev0.elapsed_time(ev1)
+    dump = scan_outputs(plan.fetch()) if args.dump_outputs and rank == 0 else None
     plan.close()
 
     # ---------------- end-to-end arm through the public API with host buffers: `e2e`
@@ -343,7 +401,7 @@ def run_ours(args):
         return t, ptable, agg, wtable, [b - a for a, b in zip(tt, tt[1:])]
 
     launches_e2e = [0]
-    e2e_steps = args.e2e_steps if args.e2e_steps else min(args.steps, 6)
+    e2e_steps = args.e2e_steps or args.steps
     e2e_step()
     barrier()
     t0 = time.perf_counter()
@@ -369,6 +427,9 @@ def run_ours(args):
     total_windows, total_launches, h2d_all, d2h_all = cnt.tolist()
 
     if rank == 0:
+        if dump is not None:
+            dump.update(e2e_outputs(agg, wtable, own_table))
+            write_outputs(args.dump_outputs, dump)
         folds_per_window = r + 1
         n_folds = (nwin + (1 if final else 0)) * folds_per_window
         cells = workcount.cells(W)
@@ -433,10 +494,14 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="C2x4", choices=sorted(WORKLOADS))
     ap.add_argument("--windows", type=int, default=0, help="debug: cap the windows of the record")
-    ap.add_argument("--e2e-steps", type=int, default=0, help="end-to-end steps (default: min(--steps, 6))")
+    ap.add_argument("--e2e-steps", type=int, default=0, help="end-to-end steps (default: --steps)")
     ap.add_argument("--cpu-windows", type=int, default=192, help="windows per CPU sample step")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step of each arm as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

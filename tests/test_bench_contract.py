@@ -1,9 +1,13 @@
-"""bench.py contract checks that need no GPU: the reference arm (CPU oracle on a bounded sample) prints one JSON line
-with the keys the driver reads; non-zero ranks of a torchrun launch stay silent; the clock sampler degrades cleanly."""
+"""bench.py contract checks.  Without a GPU: the reference arm (CPU oracle on a bounded sample) prints one JSON line
+with the documented keys; non-zero ranks of a torchrun launch stay silent; the clock sampler degrades cleanly.
+On the GPU: the arrays --dump-outputs writes."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -41,3 +45,25 @@ def test_clock_sampler_without_gpu():
     s.start()
     out = s.stop()
     assert "reasons" in out and "sm_mhz" in out
+
+
+@pytest.mark.gpu
+def test_dump_outputs_repeatable(tmp_path):
+    """--dump-outputs: float arrays of at most 64 MB in all, the same for two runs with the same arguments; --steps sets
+    the timed steps of both arms"""
+    runs = []
+    for k in range(2):
+        d = tmp_path / str(k)
+        p = _run(["--windows", "3000", "--steps", "2", "--warmup", "1", "--no-cpu-baseline", "--dump-outputs", str(d)])
+        assert p.returncode == 0, p.stderr[-3000:]
+        line = json.loads(p.stdout.strip().split("\n")[-1])
+        assert line["steps"] == 2 and line["e2e"]["steps"] == 2
+        runs.append({f: np.load(d / f) for f in sorted(os.listdir(d))})
+    a, b = runs
+    assert sorted(a) == sorted(b) and "scan_mfe_dcal.npy" in a and "e2e_nt_part.npy" in a
+    assert sum(x.nbytes for x in a.values()) <= 64 << 20
+    assert len(a["scan_mfe_dcal.npy"]) == 3000 and len(a["e2e_window_z.npy"]) == 3000
+    assert a["scan_shuffle_dcal.npy"].shape == (len(a["scan_sample_windows.npy"]), 100)
+    for f in a:
+        assert a[f].dtype in (np.float32, np.float64), f
+        assert np.array_equal(a[f], b[f], equal_nan=True), f
