@@ -35,6 +35,8 @@ def lib():
         L.sfo_eval.argtypes = [C.c_char_p, C.c_int, C.c_char_p, C.c_void_p]
         L.sfo_pf.argtypes = [C.c_char_p, C.c_int, C.c_char_p, C.c_void_p, C.c_int, C.c_double,
                              C.c_void_p, C.c_void_p, C.c_char_p, C.c_void_p]
+        L.sfo_pf_scaled.argtypes = [C.c_char_p, C.c_int, C.c_char_p, C.c_void_p, C.c_int, C.c_double, C.c_double,
+                                    C.c_void_p, C.c_void_p, C.c_char_p, C.c_void_p]
         L.sfo_deigan.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, C.c_void_p]
         L.sfo_fold_batch.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_void_p, C.c_int]
         L.sfo_fold_batch_fast.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_void_p, C.c_int]
@@ -84,8 +86,9 @@ def eval_structure(seq, structure, sc_stack=None):
     return lib().sfo_eval(seq.encode(), len(seq), structure.encode(), scp)
 
 
-def pf(seq, hc=None, sc_stack=None, max_span=0, temperature=37.0, want_bpp=False):
-    """-> dict(dG, ed, centroid, bpp)"""
+def pf(seq, hc=None, sc_stack=None, max_span=0, temperature=37.0, want_bpp=False, pf_scale=None):
+    """-> dict(dG, ed, centroid, bpp).  pf_scale None: the tables' per-nucleotide scale, and exp(-1.07 mfe / (kT n)) where
+    Z leaves the fp64 range with it; a number forces that scale (0: the tables') and raises if Z leaves the range."""
     L = lib()
     n = len(seq)
     dG = C.c_double()
@@ -93,8 +96,12 @@ def pf(seq, hc=None, sc_stack=None, max_span=0, temperature=37.0, want_bpp=False
     cen = C.create_string_buffer(n + 1)
     bpp = np.zeros((n, n), dtype=np.float64) if want_bpp else None
     keep, scp = _sc_ptr(sc_stack)
-    rc = L.sfo_pf(seq.encode(), n, hc.encode() if hc else None, scp, int(max_span or 0), float(temperature),
-                  C.addressof(dG), C.addressof(ed), cen, bpp.ctypes.data if want_bpp else None)
+    args = (C.addressof(dG), C.addressof(ed), cen, bpp.ctypes.data if want_bpp else None)
+    if pf_scale is None:
+        rc = L.sfo_pf(seq.encode(), n, hc.encode() if hc else None, scp, int(max_span or 0), float(temperature), *args)
+    else:
+        rc = L.sfo_pf_scaled(seq.encode(), n, hc.encode() if hc else None, scp, int(max_span or 0), float(temperature),
+                             float(pf_scale), *args)
     if rc != 0:
         raise RuntimeError("oracle pf: " + L.sfo_last_error().decode())
     return {"dG": dG.value, "ed": ed.value, "centroid": cen.value.decode(), "bpp": bpp}

@@ -1097,10 +1097,11 @@ static double exp_E_ExtLoop(const pfpar_t *q, int type, int si1, int sj1) {
     return z;
 }
 
-static int pf_core(ctx_t *c, double T, double *ensemble_dG, double *ed, char *centroid, double *bpp) {
+static int pf_core(ctx_t *c, double T, double pf_scale, double *ensemble_dG, double *ed, char *centroid, double *bpp) {
     const int n = c->n, N1 = n + 2;
     const int *S = c->S;
     pfpar_t *pp = pf_params(T);
+    const double ps = pf_scale > 0 ? pf_scale : pp->pf_scale;
     size_t sz = (size_t)N1 * N1;
     double *q = (double *)calloc(sz, sizeof(double)), *qb = (double *)calloc(sz, sizeof(double));
     double *qm = (double *)calloc(sz, sizeof(double)), *qm1 = (double *)calloc(sz, sizeof(double));
@@ -1114,7 +1115,7 @@ static int pf_core(ctx_t *c, double T, double *ensemble_dG, double *ed, char *ce
     scale[0] = 1.;
     eMLb[0] = 1.;
     for (int i = 1; i <= n + 2; i++) {
-        scale[i] = scale[i - 1] / pp->pf_scale;
+        scale[i] = scale[i - 1] / ps;
         eMLb[i] = pow(pp->expMLbase, (double)i) * scale[i];
     }
     /* q[i][j] for j<i (empty) = 1; short segments = scale */
@@ -1171,11 +1172,8 @@ static int pf_core(ctx_t *c, double T, double *ensemble_dG, double *ed, char *ce
         free(qq);
     }
     double Z = Q(1, n);
-    if (!(Z > 0) || isinf(Z) || isnan(Z)) {
-        set_err("pf overflow/underflow");
-        return -1;
-    }
-    if (ensemble_dG) *ensemble_dG = (-log(Z) - n * log(pp->pf_scale)) * pp->kT / 1000.0;
+    int out_of_range = !(Z > 0) || isinf(Z) || isnan(Z);
+    if (ensemble_dG) *ensemble_dG = (-log(Z) - n * log(ps)) * pp->kT / 1000.0;
 
     /* outside: base pair probabilities */
     double *q1k = (double *)calloc(n + 3, sizeof(double)), *qln = (double *)calloc(n + 3, sizeof(double));
@@ -1254,6 +1252,7 @@ static int pf_core(ctx_t *c, double T, double *ensemble_dG, double *ed, char *ce
             if (bpp) bpp[(size_t)(i - 1) * n + (j - 1)] = p;
         }
     if (ed) *ed = 2 * d;
+    out_of_range |= isinf(d) || isnan(d);
     if (centroid) {
         for (int i = 1; i <= n; i++) centroid[i - 1] = pt[i] == 0 ? '.' : (pt[i] > i ? '(' : ')');
         centroid[n] = 0;
@@ -1272,18 +1271,32 @@ static int pf_core(ctx_t *c, double T, double *ensemble_dG, double *ed, char *ce
     free(scale);
     free(eMLb);
     pf_params_free(pp);
-    return 0;
+    if (out_of_range) set_err("pf overflow/underflow");
+    return out_of_range ? 1 : 0;
 }
 
-int sfo_pf(const char *seq, int n, const char *hc, const int *sc_stack, int max_span, double temperature_c,
-           double *ensemble_dG, double *ed, char *centroid, double *bpp) {
+int sfo_pf_scaled(const char *seq, int n, const char *hc, const int *sc_stack, int max_span, double temperature_c,
+                  double pf_scale, double *ensemble_dG, double *ed, char *centroid, double *bpp) {
     ctx_t c;
     if (sfo_set_temperature(temperature_c)) return -1;
     if (ctx_init(&c, seq, n, hc, sc_stack, max_span)) return -1;
     if (bpp) memset(bpp, 0, sizeof(double) * (size_t)n * n);
-    int rc = pf_core(&c, temperature_c, ensemble_dG, ed, centroid, bpp);
+    int rc = pf_core(&c, temperature_c, pf_scale, ensemble_dG, ed, centroid, bpp);
     ctx_free(&c);
-    return rc;
+    return rc ? -1 : 0;
+}
+
+int sfo_pf(const char *seq, int n, const char *hc, const int *sc_stack, int max_span, double temperature_c,
+           double *ensemble_dG, double *ed, char *centroid, double *bpp) {
+    int rc = sfo_pf_scaled(seq, n, hc, sc_stack, max_span, temperature_c, 0, ensemble_dG, ed, centroid, bpp);
+    if (rc == 0) return 0;
+    /* Z (or the outside pass) left the fp64 range under the fixed per-nucleotide scale: ViennaRNA's exp_params_rescale
+     * rule, the scale from the MFE under the same constraints, pf_scale = exp(-1.07 mfe / (kT n)) */
+    int e = sfo_mfe(seq, n, hc, sc_stack, max_span, NULL);
+    if (e >= SFO_INF) return -1;
+    double kT = (temperature_c + K0) * GASCONST;
+    return sfo_pf_scaled(seq, n, hc, sc_stack, max_span, temperature_c, exp(-1.07 * e * 10. / (kT * n)), ensemble_dG, ed,
+                         centroid, bpp);
 }
 
 /* Boltzmann weight (unscaled) of one structure under the PF energy model -- brute-force check of pf_core */
@@ -1374,7 +1387,7 @@ static void *worker(void *arg) {
             ctx_init(&c, jb->seqs + (size_t)k * jb->len, jb->len, NULL, NULL, 0);
             if (jb->mode == 0)
                 jb->e[k] = mfe_core(&c, NULL, 0);
-            else if (pf_core(&c, 37.0, jb->dG ? jb->dG + k : NULL, jb->ed + k,
+            else if (pf_core(&c, 37.0, 0, jb->dG ? jb->dG + k : NULL, jb->ed + k,
                              jb->cen ? jb->cen + (size_t)k * (jb->len + 1) : NULL, NULL))
                 jb->bad = 1;
             ctx_free(&c);

@@ -41,6 +41,11 @@ int sfo_eval(const char *seq, int n, const char *structure, const int *sc_stack)
  * bpp: NULL or n*n doubles (row i-1, col j-1, i<j).  Returns 0 on success. */
 int sfo_pf(const char *seq, int n, const char *hc, const int *sc_stack, int max_span,
            double temperature_c, double *ensemble_dG, double *ed, char *centroid, double *bpp);
+/* sfo_pf first uses the fixed per-nucleotide scale of the tables (ViennaRNA's default pf_scale); where Z or the outside
+ * pass leaves the fp64 range it computes again with exp_params_rescale's scale exp(-1.07 mfe / (kT n)), mfe under the
+ * same constraints.  sfo_pf_scaled uses `pf_scale` (> 0; 0 = the default) and returns -1 if the range is left. */
+int sfo_pf_scaled(const char *seq, int n, const char *hc, const int *sc_stack, int max_span, double temperature_c,
+                  double pf_scale, double *ensemble_dG, double *ed, char *centroid, double *bpp);
 
 /* Boltzmann weight of one structure under the PF model (brute-force checks) */
 double sfo_eval_weight(const char *seq, int n, const char *structure, double T);

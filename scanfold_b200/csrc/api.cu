@@ -268,6 +268,39 @@ struct PfWork {
     }
 };
 
+// The PF kernels scale every nucleotide by the tables' fixed pf_scale (ViennaRNA's default).  Z of a strongly folding
+// window can leave the fp64 range under it (GC-rich windows of 400 nt at 37 C, 300 nt at 10 C): the kernels then
+// write a non-finite dG or ED and count the fold.  Such a window is folded again on pf.cu with the scale ViennaRNA's
+// exp_params_rescale derives from the window's MFE under the constraints the partition function sees,
+// pf_scale = exp(-1.07 mfe / (kT n)); the results do not depend on the scale beyond rounding.  One window per call
+// (they are rare); the outputs of `L` are overwritten.  Tables must be at `temperature`.
+void pf_rescaled_retry(PfLaunch L, double temperature, FoldWork &fw, cudaStream_t st) {
+    DevBuf<int32_t> d_e;
+    d_e.alloc(1);
+    MfeLaunch M{};
+    M.seqs = L.seqs;
+    M.hc = L.hc;
+    M.hc_simple = L.hc_simple;
+    M.sc = L.sc;
+    M.n_fold = 1;
+    M.W = L.W;
+    M.max_span = L.max_span;
+    M.e_out = d_e.p;
+    if ((!L.hc || L.hc_simple) && L.max_span <= 0)
+        fw.launch_energy_only(M, st, nullptr);
+    else
+        fw.launch_general(M, st, nullptr);
+    int32_t e = 0;
+    CK(cudaMemcpyAsync(&e, d_e.p, sizeof e, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    const double kT = (temperature + 273.15) * 1.98717;
+    L.n_fold = 1;
+    L.pf_scale = std::exp(-1.07 * e * 10. / (kT * L.W));
+    L.n_out_of_range = nullptr;
+    launch_pf(L, g_ctx.d_mfe, g_ctx.d_pf, g_ctx.n_sm, st, nullptr);
+    CK(cudaGetLastError());
+}
+
 }  // namespace
 
 // =================================================================================================
@@ -283,6 +316,7 @@ struct sfb_scan_plan {
     DevBuf<int32_t> mfe, nat_unc, shuf_e, e_tmp;
     DevBuf<int16_t> pair_tbl, centroid;
     DevBuf<double> ed, dG;
+    DevBuf<int32_t> n_out_of_range;   // PF windows whose Z left the fp64 range in the last run (see pf_rescaled_retry)
     DevBuf<uint8_t> shuf_all;  // only when shuffles_out requested at fetch time (kept per chunk -> full)
     FoldWork fw;
     PfWork pw;
@@ -547,6 +581,31 @@ int sfb_pf_batch(const uint8_t *seqs, int n_seq, int len, const sfb_model *model
         if (bpp)
             CK(cudaMemcpyAsync(bpp, d_bpp.p, sizeof(double) * d_bpp.n, cudaMemcpyDeviceToHost, g_ctx.stream));
         CK(cudaStreamSynchronize(g_ctx.stream));
+        FoldWork fw;   // prepared on the first window that needs the retry
+        for (int k = 0, prepared = 0; k < n_seq; k++) {
+            if (std::isfinite(ensemble_dG[k]) && std::isfinite(ed[k])) continue;
+            if (!prepared++) fw.prepare(len, 1);
+            PfLaunch R = L;
+            R.seqs = d_seq.p + (size_t)k * len;
+            R.hc = hc ? d_hc.p + (size_t)k * len : nullptr;
+            R.sc = sc ? d_sc.p + (size_t)k * (len + 1) : nullptr;
+            R.dG = d_dG.p + k;
+            R.ed = d_ed.p + k;
+            R.centroid = d_cen.p + (size_t)k * len;
+            R.bpp = bpp ? d_bpp.p + (size_t)k * len * len : nullptr;
+            if (bpp) CK(cudaMemsetAsync(R.bpp, 0, sizeof(double) * len * len, g_ctx.stream));
+            pf_rescaled_retry(R, model ? model->temperature : 37.0, fw, g_ctx.stream);
+            CK(cudaMemcpyAsync(ensemble_dG + k, R.dG, sizeof(double), cudaMemcpyDeviceToHost, g_ctx.stream));
+            CK(cudaMemcpyAsync(ed + k, R.ed, sizeof(double), cudaMemcpyDeviceToHost, g_ctx.stream));
+            CK(cudaMemcpyAsync(centroid_tbl + (size_t)k * len, R.centroid, sizeof(int16_t) * len, cudaMemcpyDeviceToHost,
+                               g_ctx.stream));
+            if (bpp)
+                CK(cudaMemcpyAsync(bpp + (size_t)k * len * len, R.bpp, sizeof(double) * len * len, cudaMemcpyDeviceToHost,
+                                   g_ctx.stream));
+            CK(cudaStreamSynchronize(g_ctx.stream));
+            if (!(std::isfinite(ensemble_dG[k]) && std::isfinite(ed[k])))
+                return fail(SFB_E_RANGE, "partition function of fold " + std::to_string(k) + " out of the fp64 range after rescaling");
+        }
         return 0;
     } catch (const CudaError &e) {
         return fail(SFB_E_CUDA, e.what());
@@ -612,6 +671,7 @@ int sfb_scan_plan_create(const sfb_scan_args *args, sfb_scan_plan **plan_out) {
         P->centroid.alloc((size_t)std::max(n, 1) * a.W);
         P->ed.alloc(std::max(n, 1));
         P->dG.alloc(std::max(n, 1));
+        P->n_out_of_range.alloc(1);
         CK(cudaMemset(P->centroid.p, 0, sizeof(int16_t) * P->centroid.n));
         CK(cudaMemset(P->ed.p, 0, sizeof(double) * P->ed.n));
         CK(cudaMemset(P->dG.p, 0, sizeof(double) * P->dG.n));
@@ -656,6 +716,57 @@ __global__ void copy_last_slot_kernel(int32_t *mfe, int16_t *pair_tbl, int16_t *
     }
 }
 
+// The slots of the last run whose PF left the fp64 range, again with a per-window scale (pf_rescaled_retry).  A regular
+// window is gathered from the record with its constraint slice; the final-window slot either re-ran pf() on the last
+// regular window with its soft constraints or copied that window's results (Q5), and follows it.
+static void pf_retry_out_of_range(sfb_scan_plan *P) {
+    const sfb_scan_args &a = P->a;
+    const int n = P->n_slots, W = a.W;
+    cudaStream_t st = g_ctx.stream;
+    ensure_temperature(a.model.temperature);
+    std::vector<double> dG(n), ed(n);
+    CK(cudaMemcpyAsync(dG.data(), P->dG.p, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(ed.data(), P->ed.p, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    DevBuf<uint8_t> seq, hc;
+    DevBuf<int32_t> sc;
+    seq.alloc(W);
+    if (a.hc) hc.alloc(W);
+    if (a.react) sc.alloc(W + 1);
+    for (int s = 0; s < n; s++) {
+        if (std::isfinite(dG[s]) && std::isfinite(ed[s])) continue;
+        const bool final_slot = a.final_window && s == n - 1;
+        if (final_slot && !a.react) {
+            copy_last_slot_kernel<<<(W + 127) / 128, 128, 0, st>>>(P->mfe.p, P->pair_tbl.p, P->centroid.p, P->ed.p, P->dG.p,
+                                                                   s - 1, s, W, 1);
+            CK(cudaGetLastError());
+            continue;
+        }
+        const int w = a.first_window + (final_slot ? s - 1 : s);
+        PfLaunch L{};
+        launch_gather_windows(P->seq.p, a.L, W, a.step, w, 1, 0, seq.p, st, nullptr);
+        L.seqs = seq.p;
+        if (a.hc && !final_slot) {
+            launch_slice_hc(P->hc.p, a.L, W, a.step, w, 1, 0, hc.p, st, nullptr);
+            L.hc = hc.p;
+            L.hc_simple = P->hc_simple;
+        }
+        if (final_slot) {
+            launch_slice_sc(P->es1.p, a.L, W, a.step, w, 1, 0, sc.p, st, nullptr);
+            L.sc = sc.p;
+        }
+        L.W = W;
+        L.max_span = a.model.max_bp_span;
+        L.dG = P->dG.p + s;
+        L.ed = P->ed.p + s;
+        L.centroid = P->centroid.p + (size_t)s * W;
+        L.gscratch = P->pw.scratch.p;
+        L.gscratch_per_cta = (long long)P->pw.per_cta;
+        pf_rescaled_retry(L, a.model.temperature, P->fw, st);
+    }
+    CK(cudaStreamSynchronize(st));
+}
+
 int sfb_scan_plan_run(sfb_scan_plan *P, float *ms_total, float *ms_mfe, int32_t *n_launches_out) {
     std::lock_guard<std::mutex> lk(g_mu);
     if (!P) return fail(SFB_E_ARG, "null plan");
@@ -674,6 +785,7 @@ int sfb_scan_plan_run(sfb_scan_plan *P, float *ms_total, float *ms_mfe, int32_t 
         CK(cudaEventCreate(&ep1));
         float mfe_ms = 0.f, shuf_ms = 0.f, pf_ms = 0.f;
         CK(cudaEventRecord(ev0, st));
+        CK(cudaMemsetAsync(P->n_out_of_range.p, 0, sizeof(int32_t), st));
         const int n = P->n_slots, r = a.r, W = a.W;
         const double t_model = a.model.temperature, t_bg = a.background_temperature != 0. ? a.background_temperature : t_model;
         for (int c0 = 0, cn = 0; c0 < n; c0 += cn) {
@@ -776,6 +888,7 @@ int sfb_scan_plan_run(sfb_scan_plan *P, float *ms_total, float *ms_mfe, int32_t 
                 L.centroid = P->centroid.p + (size_t)c0 * W;
                 L.gscratch = P->pw.scratch.p;
                 L.gscratch_per_cta = (long long)P->pw.per_cta;
+                L.n_out_of_range = P->n_out_of_range.p;
                 launch_pf(L, g_ctx.d_mfe, g_ctx.d_pf, g_ctx.n_sm, st, &n_launch);
             }
             CK(cudaEventRecord(ep1, st));
@@ -795,6 +908,7 @@ int sfb_scan_plan_run(sfb_scan_plan *P, float *ms_total, float *ms_mfe, int32_t 
                     L.centroid = P->centroid.p + (size_t)fin * W;
                     L.gscratch = P->pw.scratch.p;
                     L.gscratch_per_cta = (long long)P->pw.per_cta;
+                    L.n_out_of_range = P->n_out_of_range.p;
                     launch_pf(L, g_ctx.d_mfe, g_ctx.d_pf, g_ctx.n_sm, st, &n_launch);
                     copy_pf = 0;
                 }
@@ -811,9 +925,13 @@ int sfb_scan_plan_run(sfb_scan_plan *P, float *ms_total, float *ms_mfe, int32_t 
             CK(cudaEventElapsedTime(&ms, em1, ep1));
             pf_ms += ms;
         }
+        int32_t n_out_of_range = 0;
+        if (a.want_pf)
+            CK(cudaMemcpyAsync(&n_out_of_range, P->n_out_of_range.p, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
         CK(cudaEventRecord(ev1, st));
         CK(cudaEventSynchronize(ev1));
         CK(cudaGetLastError());
+        if (n_out_of_range > 0) pf_retry_out_of_range(P);
         float tot = 0.f;
         CK(cudaEventElapsedTime(&tot, ev0, ev1));
         if (ms_total) *ms_total = tot;

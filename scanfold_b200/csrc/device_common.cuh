@@ -92,6 +92,8 @@ struct PfLaunch {
     double *gscratch;     // per-CTA workspace
     long long gscratch_per_cta;  // doubles
     int hc_simple;        // hc holds no '(' ')' : per-nucleotide flags only, which pf2 folds in
+    double pf_scale;      // 0: the tables' per-nucleotide scale; > 0: this one (range retry, pf.cu only)
+    int *n_out_of_range;  // NULL or a counter: +1 per fold whose dG or ED is not finite (Z left the fp64 range)
 };
 
 void launch_mfe(const MfeLaunch &L, const MfeTables *d_tab, int n_sm, cudaStream_t stream, int *n_launches);

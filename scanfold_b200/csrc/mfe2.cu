@@ -28,6 +28,7 @@ namespace sfb {
 namespace {
 
 constexpr int INF16 = 16000;
+constexpr int TABLE_ENV16 = 2000;   // |table entry| the int16 arithmetic accepts (DESIGN §2)
 constexpr int FIN16 = 4000;
 constexpr int LOW16 = -12000;
 constexpr int ROLL = 34;   // rows d-32 .. d+1 are live while a pair of diagonals (d, d+1) is computed
@@ -444,20 +445,27 @@ int mfe2_grid_size(int n_sm, int n_fold) {
 
 void mfe2_upload_tables(const MfeTables &M) {
     static Tab2 h;
+    // every entry below is stored as int16: a table value outside the envelope (INF entries of the stack / mismatch
+    // tables included, which (short) would wrap) declines the table, and the int32 kernel folds instead
+    bool fit = true;
+    auto s16 = [&fit](int v) {
+        fit = fit && v >= -TABLE_ENV16 && v <= TABLE_ENV16;
+        return (short)v;
+    };
     auto mm = [](int t, int a, int b) { return (t * 5 + a) * 5 + b; };
     static const int rt[8] = {0, 2, 1, 4, 3, 6, 5, 7};
     for (int a = 0; a < 8; a++)
-        for (int b = 0; b < 8; b++) h.stack[a * 8 + b] = (short)M.stack[a][b];
+        for (int b = 0; b < 8; b++) h.stack[a * 8 + b] = s16(M.stack[a][b]);
     for (int t = 0; t < 8; t++) {
-        h.tAU[t] = (short)(t > 2 ? M.TerminalAU : 0);
+        h.tAU[t] = s16(t > 2 ? M.TerminalAU : 0);
         h.rtype[t] = (unsigned char)rt[t];
         for (int a = 0; a < 5; a++)
             for (int b = 0; b < 5; b++) {
-                h.mmI[mm(t, a, b)] = (short)M.mismatchI[t][a][b];
-                h.mm1n[mm(t, a, b)] = (short)M.mismatch1nI[t][a][b];
-                h.mm23[mm(t, a, b)] = (short)M.mismatch23I[t][a][b];
-                h.mmH[mm(t, a, b)] = (short)M.mismatchH[t][a][b];
-                h.mlclose[mm(t, a, b)] = (short)(M.mismatchM[t][a][b] + (t > 2 ? M.TerminalAU : 0) + M.MLintern + M.MLclosing);
+                h.mmI[mm(t, a, b)] = s16(M.mismatchI[t][a][b]);
+                h.mm1n[mm(t, a, b)] = s16(M.mismatch1nI[t][a][b]);
+                h.mm23[mm(t, a, b)] = s16(M.mismatch23I[t][a][b]);
+                h.mmH[mm(t, a, b)] = s16(M.mismatchH[t][a][b]);
+                h.mlclose[mm(t, a, b)] = s16(M.mismatchM[t][a][b] + (t > 2 ? M.TerminalAU : 0) + M.MLintern + M.MLclosing);
             }
         for (int a = 0; a < 6; a++)
             for (int b = 0; b < 6; b++) {
@@ -471,17 +479,17 @@ void mfe2_upload_tables(const MfeTables &M) {
                     em = ee = M.dangle3[t][b];
                 }
                 const int au = t > 2 ? M.TerminalAU : 0;
-                h.mlstem[t * 36 + a * 6 + b] = (short)(em + au + M.MLintern);
-                h.ext[t * 36 + a * 6 + b] = (short)(ee + au);
+                h.mlstem[t * 36 + a * 6 + b] = s16(em + au + M.MLintern);
+                h.ext[t * 36 + a * 6 + b] = s16(ee + au);
             }
     }
     for (int a = 0; a < 6; a++)
         for (int b = 0; b < 6; b++) h.ptype[a * 6 + b] = (unsigned char)((a < 5 && b < 5) ? pair_type(a, b) : 0);
-    h.bulge1 = (short)M.bulge[1];
-    h.il5_ninio = (short)(M.internal_loop[5] + M.ninio);
-    h.MLbase = (short)M.MLbase;
+    h.bulge1 = s16(M.bulge[1]);
+    h.il5_ninio = s16(M.internal_loop[5] + M.ninio);
+    h.MLbase = s16(M.MLbase);
     static int sG[31][32], s1[32], sB[32], sC[32];
-    g_mfe2_ok = M.ninio >= 0 && NEAR * M.ninio >= M.max_ninio;
+    g_mfe2_ok = fit && M.ninio >= 0 && NEAR * M.ninio >= M.max_ninio;
     for (int u = 0; u <= MAXLOOP; u++) {
         sC[u] = M.internal_loop[u] < INF ? M.internal_loop[u] + M.max_ninio : INF16;
         sB[u] = M.bulge[u] < INF ? M.bulge[u] : INF16;

@@ -201,7 +201,7 @@ __global__ void __launch_bounds__(NT, SFB_PF_MINB) pf_kernel(PfLaunch L, const M
             st->expMLintern = T->expMLintern;
             st->expTermAU = T->expTermAU;
             st->kT = T->kT;
-            st->pf_scale = T->pf_scale;
+            st->pf_scale = L.pf_scale > 0. ? L.pf_scale : T->pf_scale;
             int n = 0;
             for (int u = 0; u <= MAXLOOP; u++) {
                 for (int u1 = 0; u1 <= u; u1++) {
@@ -217,8 +217,8 @@ __global__ void __launch_bounds__(NT, SFB_PF_MINB) pf_kernel(PfLaunch L, const M
             scale[0] = 1.;
             eMLb[0] = 1.;
             for (int k = 1; k < W + 4; k++) {
-                scale[k] = scale[k - 1] / T->pf_scale;
-                eMLb[k] = eMLb[k - 1] * T->expMLbase / T->pf_scale;
+                scale[k] = scale[k - 1] / st->pf_scale;
+                eMLb[k] = eMLb[k - 1] * T->expMLbase / st->pf_scale;
             }
         }
     }
@@ -597,8 +597,10 @@ __global__ void __launch_bounds__(NT, SFB_PF_MINB) pf_kernel(PfLaunch L, const M
         if (tid == 0) {
             double s = 0.;
             for (int w = 0; w < NT / 32; w++) s += red[w];
+            const double dG = (-log(Z) - W * log(st->pf_scale)) * st->kT / 1000.;
             L.ed[fold] = 2. * s;
-            L.dG[fold] = (-log(Z) - W * log(st->pf_scale)) * st->kT / 1000.;
+            L.dG[fold] = dG;
+            if (L.n_out_of_range && !(isfinite(dG) && isfinite(2. * s))) atomicAdd(L.n_out_of_range, 1);
         }
         for (int k = tid; k < W; k += NT) L.centroid[(long long)fold * W + k] = cen[k];
         __syncthreads();

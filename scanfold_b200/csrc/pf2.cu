@@ -827,8 +827,10 @@ pf2_kernel(PfLaunch L, const MfeTables *__restrict__ MT, const PfTables *__restr
         if (tid == 0) {
             double s = 0.;
             for (int w = 0; w < NW2; w++) s += sm.red[w];
+            const double dG = (-log(Z) - W * log(T->pf_scale)) * T->kT / 1000.;
             L.ed[fold] = 2. * s;
-            L.dG[fold] = (-log(Z) - W * log(T->pf_scale)) * T->kT / 1000.;
+            L.dG[fold] = dG;
+            if (L.n_out_of_range && !(isfinite(dG) && isfinite(2. * s))) atomicAdd(L.n_out_of_range, 1);
         }
         for (int k = tid; k < W; k += NT2) L.centroid[(long long)fold * W + k] = sm.cen[k];
 #ifdef SFB_PF2_TIMING
@@ -850,7 +852,8 @@ static bool &pf2_enabled() {
 void pf2_set_enabled(bool on) { pf2_enabled() = on; }
 
 bool pf2_supports(const PfLaunch &L) {
-    return pf2_enabled() && (!L.hc || L.hc_simple) && !L.sc && L.max_span <= 0 && L.W >= 2 * TURN + 4 && L.W <= P2;
+    return pf2_enabled() && (!L.hc || L.hc_simple) && !L.sc && L.max_span <= 0 && L.pf_scale <= 0. && L.W >= 2 * TURN + 4 &&
+           L.W <= P2;   // the scale is baked into g_K2 and the shared scale row: a rescaled retry runs on pf.cu
 }
 
 size_t pf2_scratch_doubles_per_cta() { return 2 * (size_t)P2 * P2; }
