@@ -168,6 +168,35 @@ int sfb_accumulate_fetch(sfb_partner_table *table, int32_t *nparts, int32_t *par
 int sfb_accumulate_launches(const sfb_partner_table *table);
 void sfb_accumulate_free(sfb_partner_table *table);
 
+/* Window-averaged base-pair probabilities (the local pair-probability view of RNAplfold -W W -L W at step 1), kept
+ * from the partition functions the scan already computes.  No reference counterpart (an additive output).
+ * p^w(i,j) is the base-pair probability of (i,j) in the partition function of regular window w: the one whose ED
+ * the scan reports (hard constraints and max_bp_span apply, soft constraints do not; the final-window slot is not a
+ * window here).  With n(i,j) / n(i) the numbers of regular windows of the record that hold both i and j / hold i:
+ *   P(i,j) = sum_w p^w(i,j) / n(i,j),   paired(i) = sum_w sum_k p^w(i,k) / n(i).
+ * A table covers the nucleotides (0-based) [first_window*step, (first_window+n_windows-1)*step + W) of a shard of
+ * windows: one row each, W int64 columns (0: sum of paired_w(i); d >= 1: sum of p^w(i,i+d)).  Every probability
+ * enters as llrint(p * 2^40), so the sums are exact: the same for any chunking, split of the scan into plans, and
+ * number of GPUs.  A window adds its probabilities once, from the run whose dG and ED are finite (a window out of the
+ * fp64 range adds them from its rescaled retry). */
+typedef struct sfb_pairprob_table sfb_pairprob_table;
+int sfb_pairprob_begin(int32_t L, int32_t W, int32_t step, int32_t first_window, int32_t n_windows,
+                       sfb_pairprob_table **table);
+/* Attach `table` to a plan before sfb_scan_plan_run: every run then adds the probabilities of the plan's regular
+ * windows to it.  The plan must compute the partition function (want_pf = 1), have the table's record length, W and
+ * step, and its windows must lie in the table's range.  The table must outlive the plan's runs. */
+int sfb_scan_plan_pairprob(sfb_scan_plan *plan, sfb_pairprob_table *table);
+/* Halo exchange between neighbouring shards (multi-GPU): copy rows [row0, row0+n_rows) out to / add them in from a
+ * DEVICE buffer of n_rows*W int64 that the caller moves with NCCL. */
+int sfb_pairprob_export(sfb_pairprob_table *table, int row0, int n_rows, int64_t *d_rows);
+int sfb_pairprob_merge(sfb_pairprob_table *table, int row0, int n_rows, const int64_t *d_rows);
+/* Reduce rows [row0, row0+n_rows) on the device: paired(i) per row (0 where no window holds i) and the pairs with
+ * P(i,j) >= cutoff (> 0), sorted by i then j; returns their number. */
+int sfb_pairprob_compact(sfb_pairprob_table *table, int row0, int n_rows, double cutoff, int64_t *n_pairs);
+/* Results of the last compact: paired [n_rows], i / j [n_pairs] 1-based record coordinates, p [n_pairs] = P(i,j). */
+int sfb_pairprob_fetch(sfb_pairprob_table *table, double *paired, int32_t *i, int32_t *j, double *p);
+void sfb_pairprob_free(sfb_pairprob_table *table);
+
 /* Roofline denominators measured on the current device (bench.py): SFB_MICROBENCH_ADDMIN = int32
  * add-min (VIADDMNMX) operations per second over all SMs; SFB_MICROBENCH_SMEM_LD32 = conflict-free
  * 32-bit shared-memory loads per second (x4 = bytes/s).  No reference counterpart. */

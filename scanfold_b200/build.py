@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.environ.get("SFB_BUILD_OUT") or os.path.join(HERE, "libscanfold_b200.so")   # SFB_BUILD_OUT: debug variants
-SOURCES = ["params.cpp", "mfe.cu", "mfe2.cu", "mfe3.cu", "mfe4.cu", "pf.cu", "pf2.cu", "shuffle.cu", "accumulate.cu", "microbench.cu", "api.cu"]
+SOURCES = ["params.cpp", "mfe.cu", "mfe2.cu", "mfe3.cu", "mfe4.cu", "pf.cu", "pf2.cu", "shuffle.cu", "accumulate.cu", "pairprob.cu", "microbench.cu", "api.cu"]
 EXTRA = os.environ.get("SFB_NVCC_EXTRA", "").split()
 NVCC_FLAGS = EXTRA + ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden"]

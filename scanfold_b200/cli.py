@@ -85,6 +85,10 @@ def build_parser():
                    help="[scanfold_b200] .npz with `shuffles` [(windows+1), r, W] uint8 to fold instead of device shuffles")
     p.add_argument("--params", type=str, default=None, help="[scanfold_b200] ViennaRNA parameter file")
     p.add_argument("--gpu", type=int, default=0, help="[scanfold_b200] CUDA device ordinal")
+    p.add_argument("--pair_probs", action="store_true",
+                   help="[scanfold_b200] also write the window-averaged base-pair probabilities of the scan's partition "
+                        "functions: <out>.pairprob.wig (probability of being paired), <out>.pairprob.txt (pairs with "
+                        "P >= 0.01) and an IGV arc track of the pairs with P >= 0.1")
     return p
 
 
@@ -258,12 +262,14 @@ def run_record(args, record_name, raw_seq, original_directory, dist=None):
             parity = allsh[w0:w1 + (1 if last else 0)]
         if rank == 0:
             print("Scanning input sequence:", read_name)
-        acc = None
+        acc = pp = None
         if w1 > w0:
+            if args.pair_probs:
+                pp = engine.PairProbTable(len(seq), W, step, w0, w1 - w0)
             shard = scan.scan_record(seq.upper(), W, step, r, shuffle_type=str(args.type), seed=args.seed,
                                      parity_shuffles=parity, temperature=float(args.t), max_span=args.span or 0, hc=hc,
                                      react=react, shape_m=args.m, shape_b=args.b, first_window=w0, n_windows=w1 - w0,
-                                     final_window=last)
+                                     final_window=last, pairprob=pp)
             shard.alln = scan.all_n_windows(seq, W, step, w0, w1 - w0)      # Q10: tested on the record as given
             if last and scan.final_window_all_n(seq, W):
                 shard.final = None                                          # the final-window block appends nothing (:719-726)
@@ -276,6 +282,13 @@ def run_record(args, record_name, raw_seq, original_directory, dist=None):
         finally:
             if acc is not None:
                 acc.close()
+        pairprob = None
+        if args.pair_probs:
+            try:
+                pairprob = multigpu.pairprob_distributed(pp, W, step, rank, world, dist, total, engine.PAIR_CUTOFF)
+            finally:
+                if pp is not None:
+                    pp.close()
         # every rank aggregates the nucleotides it owns; rank 0 gets the per-nucleotide results and the log text
         aggregated = multigpu.aggregate_distributed(own_table, seq, rank, world, dist, by_ed=bool(args.by_ed), with_logs=True)
         table = multigpu.gather_window_tables(shard, rank, world, dist, with_shuffle_energies=bool(args.print_random))
@@ -288,6 +301,8 @@ def run_record(args, record_name, raw_seq, original_directory, dist=None):
         pipeline.write_fold_outputs(seq, None, names, minz, step, by_ed=bool(args.by_ed), competition=int(args.c),
                                     zscores=pipeline.zscore_total(table), filter_value=int(args.f),
                                     input_filename=args.filename, aggregated=aggregated)
+        if pairprob is not None:
+            pipeline.write_pairprob_outputs(pairprob, names, W, step, total)
         if args.global_refold:
             global_refold(seq, names, args.name, float(args.t), args.span or 0)
         # structure extraction: refold every top-level helix of the Zavg < -2 structure (ScanFold.py:1557-1781)

@@ -145,8 +145,13 @@ void launch_accum_count(const AccumDense &D, int row0, int n_rows, int32_t *npar
                         cudaStream_t stream, int *n_launches) {
     if (n_rows <= 0) return;
     count_kernel<<<(n_rows + 127) / 128, 128, 0, stream>>>(D, row0, n_rows, nparts);
-    scan_kernel<<<1, 1024, 0, stream>>>(nparts, n_rows, offsets);
-    if (n_launches) (*n_launches) += 2;
+    if (n_launches) (*n_launches)++;
+    launch_exclusive_scan(nparts, n_rows, offsets, stream, n_launches);
+}
+
+void launch_exclusive_scan(const int32_t *counts, int n, long long *offsets, cudaStream_t stream, int *n_launches) {
+    scan_kernel<<<1, 1024, 0, stream>>>(counts, n, offsets);
+    if (n_launches) (*n_launches)++;
 }
 
 void launch_accum_emit(const AccumDense &D, int row0, int n_rows, const long long *offsets, int32_t *partner,

@@ -261,8 +261,8 @@ struct FoldWork {  // device scratch for one MFE launch
 struct PfWork {
     DevBuf<double> scratch;
     size_t per_cta = 0;
-    void prepare(int W, int n_fold) {
-        per_cta = pf_scratch_doubles_per_cta(W);
+    void prepare(int W, int n_fold, bool pairprob = false) {
+        per_cta = pf_scratch_doubles_per_cta(W, pairprob);
         size_t need = per_cta * (size_t)pf_grid_size(W, g_ctx.n_sm, n_fold);
         if (need > scratch.n) scratch.alloc(need);
     }
@@ -274,7 +274,7 @@ struct PfWork {
 // exp_params_rescale derives from the window's MFE under the constraints the partition function sees,
 // pf_scale = exp(-1.07 mfe / (kT n)); the results do not depend on the scale beyond rounding.  One window per call
 // (they are rare); the outputs of `L` are overwritten.  Tables must be at `temperature`.
-void pf_rescaled_retry(PfLaunch L, double temperature, FoldWork &fw, cudaStream_t st) {
+void pf_rescaled_retry(PfLaunch L, double temperature, FoldWork &fw, cudaStream_t st, const PairProbCommit &pp = {}) {
     DevBuf<int32_t> d_e;
     d_e.alloc(1);
     MfeLaunch M{};
@@ -297,13 +297,24 @@ void pf_rescaled_retry(PfLaunch L, double temperature, FoldWork &fw, cudaStream_
     L.n_fold = 1;
     L.pf_scale = std::exp(-1.07 * e * 10. / (kT * L.W));
     L.n_out_of_range = nullptr;
-    launch_pf(L, g_ctx.d_mfe, g_ctx.d_pf, g_ctx.n_sm, st, nullptr);
+    launch_pf(L, g_ctx.d_mfe, g_ctx.d_pf, g_ctx.n_sm, st, nullptr, pp);
     CK(cudaGetLastError());
 }
 
 }  // namespace
 
 // =================================================================================================
+struct sfb_pairprob_table {
+    PairProbDense D{};
+    int L = 0, first_window = 0, n_windows = 0;   // the record and the shard of windows the table covers
+    DevBuf<long long> cells;
+    DevBuf<double> paired, prob;
+    DevBuf<int32_t> npairs, pi, pj;
+    DevBuf<long long> offsets;
+    int c_rows = 0;
+    long long n_pairs = -1;
+};
+
 struct sfb_scan_plan {
     sfb_scan_args a;
     int n_slots = 0;        // n_windows + final
@@ -321,6 +332,7 @@ struct sfb_scan_plan {
     FoldWork fw;
     PfWork pw;
     bool keep_shuffles = false;
+    sfb_pairprob_table *pp = nullptr;   // sfb_scan_plan_pairprob: every run adds its regular windows' probabilities
     float stage_ms[4] = {0.f, 0.f, 0.f, 0.f};   // last run: gather + shuffles, MFE, PF, rest
 };
 
@@ -762,7 +774,10 @@ static void pf_retry_out_of_range(sfb_scan_plan *P) {
         L.centroid = P->centroid.p + (size_t)s * W;
         L.gscratch = P->pw.scratch.p;
         L.gscratch_per_cta = (long long)P->pw.per_cta;
-        pf_rescaled_retry(L, a.model.temperature, P->fw, st);
+        PairProbCommit pp{};
+        if (P->pp && !final_slot)   // the first attempt added nothing: this run is the window's only contribution
+            pp = PairProbCommit{P->pp->cells.p, (long long)w * a.step - P->pp->D.nt0, a.step};
+        pf_rescaled_retry(L, a.model.temperature, P->fw, st, pp);
     }
     CK(cudaStreamSynchronize(st));
 }
@@ -889,7 +904,9 @@ int sfb_scan_plan_run(sfb_scan_plan *P, float *ms_total, float *ms_mfe, int32_t 
                 L.gscratch = P->pw.scratch.p;
                 L.gscratch_per_cta = (long long)P->pw.per_cta;
                 L.n_out_of_range = P->n_out_of_range.p;
-                launch_pf(L, g_ctx.d_mfe, g_ctx.d_pf, g_ctx.n_sm, st, &n_launch);
+                PairProbCommit pp{};
+                if (P->pp) pp = PairProbCommit{P->pp->cells.p, (long long)(a.first_window + c0) * a.step - P->pp->D.nt0, a.step};
+                launch_pf(L, g_ctx.d_mfe, g_ctx.d_pf, g_ctx.n_sm, st, &n_launch, pp);
             }
             CK(cudaEventRecord(ep1, st));
             if (has_final) {
@@ -1182,6 +1199,154 @@ int sfb_accumulate_fetch(sfb_partner_table *T, int32_t *nparts, int32_t *partner
 }
 
 int sfb_accumulate_launches(const sfb_partner_table *T) { return T ? T->n_launches : 0; }
+
+// -------------------------------------------------------------------------------------------------
+int sfb_pairprob_begin(int32_t L, int32_t W, int32_t step, int32_t first_window, int32_t n_windows,
+                       sfb_pairprob_table **out) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    if (!g_ctx.ready) return fail(SFB_E_STATE, "sfb_init has not been called");
+    if (!out) return fail(SFB_E_ARG, "null argument");
+    if (L < 1 || W < 1 || W > L || step < 1 || n_windows < 1 || first_window < 0)
+        return fail(SFB_E_ARG, "sfb_pairprob_begin: bad geometry");
+    if (W > MAX_W) return fail(SFB_E_RANGE, "window exceeds MAX_W");
+    const int total = (L - W) / step + 1;
+    if (first_window + n_windows > total) return fail(SFB_E_ARG, "window range exceeds the record");
+    try {
+        CK(cudaSetDevice(g_ctx.device));
+        auto *T = new sfb_pairprob_table();
+        std::unique_ptr<sfb_pairprob_table> guard(T);
+        T->L = L;
+        T->first_window = first_window;
+        T->n_windows = n_windows;
+        T->D.nt0 = first_window * step;
+        T->D.n_nt = (n_windows - 1) * step + W;
+        T->D.W = W;
+        T->D.step = step;
+        T->D.n_windows = total;
+        T->cells.alloc((size_t)T->D.n_nt * W);
+        T->D.cells = T->cells.p;
+        CK(cudaMemsetAsync(T->cells.p, 0, sizeof(long long) * T->cells.n, g_ctx.stream));
+        CK(cudaStreamSynchronize(g_ctx.stream));
+        *out = guard.release();
+        return 0;
+    } catch (const CudaError &e) {
+        return fail(SFB_E_CUDA, e.what());
+    }
+}
+
+int sfb_scan_plan_pairprob(sfb_scan_plan *P, sfb_pairprob_table *T) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    if (!P || !T) return fail(SFB_E_ARG, "null argument");
+    const sfb_scan_args &a = P->a;
+    if (!a.want_pf) return fail(SFB_E_ARG, "sfb_scan_plan_pairprob: the plan computes no partition function (want_pf = 0)");
+    if (a.L != T->L || a.W != T->D.W || a.step != T->D.step)
+        return fail(SFB_E_ARG, "sfb_scan_plan_pairprob: record length, window or step differ from the table's");
+    if (a.first_window < T->first_window || a.first_window + a.n_windows > T->first_window + T->n_windows)
+        return fail(SFB_E_ARG, "sfb_scan_plan_pairprob: the plan's windows lie outside the table's range");
+    try {
+        CK(cudaSetDevice(g_ctx.device));
+        P->pw.prepare(a.W, P->chunk + 1, true);   // pf2 stages the probabilities of a fold in its scratch
+        P->pp = T;
+        return 0;
+    } catch (const CudaError &e) {
+        return fail(SFB_E_CUDA, e.what());
+    }
+}
+
+static int check_pp_rows(const sfb_pairprob_table *T, int row0, int n_rows) {
+    if (!T) return fail(SFB_E_ARG, "null table");
+    if (row0 < 0 || n_rows < 0 || row0 + n_rows > T->D.n_nt) return fail(SFB_E_ARG, "row range outside the table");
+    return 0;
+}
+
+int sfb_pairprob_export(sfb_pairprob_table *T, int row0, int n_rows, int64_t *d_rows) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    if (int rc = check_pp_rows(T, row0, n_rows)) return rc;
+    if (!d_rows) return fail(SFB_E_ARG, "null buffer");
+    try {
+        CK(cudaSetDevice(g_ctx.device));
+        const size_t n = (size_t)n_rows * T->D.W;
+        if (n)
+            CK(cudaMemcpyAsync(d_rows, T->cells.p + (size_t)row0 * T->D.W, n * 8, cudaMemcpyDeviceToDevice, g_ctx.stream));
+        CK(cudaStreamSynchronize(g_ctx.stream));
+        return 0;
+    } catch (const CudaError &e) {
+        return fail(SFB_E_CUDA, e.what());
+    }
+}
+
+int sfb_pairprob_merge(sfb_pairprob_table *T, int row0, int n_rows, const int64_t *d_rows) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    if (int rc = check_pp_rows(T, row0, n_rows)) return rc;
+    if (!d_rows) return fail(SFB_E_ARG, "null buffer");
+    try {
+        CK(cudaSetDevice(g_ctx.device));
+        launch_pairprob_merge(T->D, row0, n_rows, (const long long *)d_rows, g_ctx.stream, nullptr);
+        CK(cudaGetLastError());
+        CK(cudaStreamSynchronize(g_ctx.stream));
+        return 0;
+    } catch (const CudaError &e) {
+        return fail(SFB_E_CUDA, e.what());
+    }
+}
+
+int sfb_pairprob_compact(sfb_pairprob_table *T, int row0, int n_rows, double cutoff, int64_t *n_pairs) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    if (int rc = check_pp_rows(T, row0, n_rows)) return rc;
+    if (!n_pairs) return fail(SFB_E_ARG, "null argument");
+    if (!(cutoff > 0.)) return fail(SFB_E_ARG, "sfb_pairprob_compact: cutoff must be positive");
+    try {
+        CK(cudaSetDevice(g_ctx.device));
+        cudaStream_t st = g_ctx.stream;
+        T->c_rows = n_rows;
+        T->paired.alloc(std::max(n_rows, 1));
+        T->npairs.alloc(std::max(n_rows, 1));
+        T->offsets.alloc((size_t)n_rows + 1);
+        launch_pairprob_count(T->D, row0, n_rows, cutoff, T->paired.p, T->npairs.p, T->offsets.p, st, nullptr);
+        long long total = 0;
+        if (n_rows > 0) CK(cudaMemcpyAsync(&total, T->offsets.p + n_rows, 8, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        const size_t m = (size_t)std::max<long long>(total, 1);
+        T->pi.alloc(m);
+        T->pj.alloc(m);
+        T->prob.alloc(m);
+        if (total > 0)
+            launch_pairprob_emit(T->D, row0, n_rows, cutoff, T->offsets.p, T->pi.p, T->pj.p, T->prob.p, st, nullptr);
+        CK(cudaGetLastError());
+        CK(cudaStreamSynchronize(st));
+        T->n_pairs = total;
+        *n_pairs = total;
+        return 0;
+    } catch (const CudaError &e) {
+        return fail(SFB_E_CUDA, e.what());
+    }
+}
+
+int sfb_pairprob_fetch(sfb_pairprob_table *T, double *paired, int32_t *i, int32_t *j, double *p) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    if (!T || T->n_pairs < 0) return fail(SFB_E_STATE, "sfb_pairprob_compact has not been called");
+    if ((T->c_rows && !paired) || (T->n_pairs && (!i || !j || !p))) return fail(SFB_E_ARG, "null buffer");
+    try {
+        CK(cudaSetDevice(g_ctx.device));
+        cudaStream_t st = g_ctx.stream;
+        const size_t m = (size_t)T->n_pairs;
+        if (T->c_rows) CK(cudaMemcpyAsync(paired, T->paired.p, sizeof(double) * T->c_rows, cudaMemcpyDeviceToHost, st));
+        if (m) {
+            CK(cudaMemcpyAsync(i, T->pi.p, 4 * m, cudaMemcpyDeviceToHost, st));
+            CK(cudaMemcpyAsync(j, T->pj.p, 4 * m, cudaMemcpyDeviceToHost, st));
+            CK(cudaMemcpyAsync(p, T->prob.p, 8 * m, cudaMemcpyDeviceToHost, st));
+        }
+        CK(cudaStreamSynchronize(st));
+        return 0;
+    } catch (const CudaError &e) {
+        return fail(SFB_E_CUDA, e.what());
+    }
+}
+
+void sfb_pairprob_free(sfb_pairprob_table *T) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    delete T;
+}
 
 void sfb_accumulate_free(sfb_partner_table *T) {
     std::lock_guard<std::mutex> lk(g_mu);

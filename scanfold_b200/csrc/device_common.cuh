@@ -95,6 +95,14 @@ struct PfLaunch {
     double pf_scale;      // 0: the tables' per-nucleotide scale; > 0: this one (range retry, pf.cu only)
     int *n_out_of_range;  // NULL or a counter: +1 per fold whose dG or ED is not finite (Z left the fp64 range)
 };
+// Where a PF launch commits its probabilities (pairprob.cu), a kernel argument of its own so that the PfLaunch of the
+// default path keeps its layout.  table NULL: none.  A fold whose dG and ED come out finite adds its probabilities to
+// rows row0 + fold * step + i of the table (W columns each, see PairProbDense); a fold out of the fp64 range adds nothing.
+struct PairProbCommit {
+    long long *table;
+    long long row0;
+    int step;
+};
 
 void launch_mfe(const MfeLaunch &L, const MfeTables *d_tab, int n_sm, cudaStream_t stream, int *n_launches);
 size_t mfe_scratch_ints_per_cta(int W, int *mats_in_gmem);
@@ -121,15 +129,15 @@ void launch_mfe4(const MfeLaunch &L, const MfeTables *d_tab, const int32_t *d_hp
                  int32_t *pair32, int n_sm, cudaStream_t stream, int *n_launches);
 
 void launch_pf(const PfLaunch &L, const MfeTables *d_mfe, const PfTables *d_pf, int n_sm, cudaStream_t stream,
-               int *n_launches);
-size_t pf_scratch_doubles_per_cta(int W);
+               int *n_launches, const PairProbCommit &pp = PairProbCommit{});
+size_t pf_scratch_doubles_per_cta(int W, bool pairprob = false);
 // second-generation partition function (pf2.cu): unconstrained windows up to 120 nt, shared-memory resident
 bool pf2_supports(const PfLaunch &L);
 void pf2_set_enabled(bool on);
-size_t pf2_scratch_doubles_per_cta();
+size_t pf2_scratch_doubles_per_cta(bool pairprob);
 void pf2_upload_tables(const PfTables &q);
 void launch_pf2(const PfLaunch &L, const MfeTables *d_mfe, const PfTables *d_pf, int n_sm, cudaStream_t stream,
-                int *n_launches);
+                int *n_launches, const PairProbCommit &pp);
 int pf_grid_size(int W, int n_sm, int n_fold);
 
 constexpr int SHUFFLE_MONO = 0, SHUFFLE_DI = 1;
@@ -172,8 +180,47 @@ void launch_accum_merge(const AccumDense &D, int row0, int n_rows, const int32_t
 // per-nucleotide partner counts for rows [row0, row0 + n_rows) -> nparts[n_rows]; offsets[n_rows + 1] = exclusive scan
 void launch_accum_count(const AccumDense &D, int row0, int n_rows, int32_t *nparts, long long *offsets,
                         cudaStream_t stream, int *n_launches);
+// exclusive scan of n counts -> offsets[n + 1] (one CTA)
+void launch_exclusive_scan(const int32_t *counts, int n, long long *offsets, cudaStream_t stream, int *n_launches);
 void launch_accum_emit(const AccumDense &D, int row0, int n_rows, const long long *offsets, int32_t *partner,
                        int32_t *count, int32_t *first_seen, long long *sums, long long n_entries, cudaStream_t stream,
                        int *n_launches);
+
+// Window-averaged base-pair probabilities (pairprob.cu): a dense table over the nucleotides a shard of windows touches,
+// W int64 columns per row.  Column 0 of row i sums paired_w(i) = sum_k p^w(i,k) over the windows, column d >= 1 sums
+// p^w(i, i+d).  Every term enters as the integer llrint(p * 2^40), so the sums are exact and do not depend on the
+// order in which windows, chunks, parts of a scan or GPUs add them.
+constexpr double PP_UNIT = 1099511627776.0;   // 2^40
+struct PairProbDense {
+    int nt0, n_nt, W, step, n_windows;   // rows = nucleotides [nt0, nt0 + n_nt) (0-based); n_windows of the whole record
+    long long *cells;                    // [n_nt][W]
+};
+
+// The PF kernels' commit of one fold: row i (window coordinates) of the fold's probabilities p(k, l) (k < l) into the
+// table rows at `rows` (row i at rows + i * W).  The per-nucleotide sum is formed in a fixed order from the same
+// integers that go into the pair columns; the adds are integer reductions.
+template <class P>
+__device__ __forceinline__ void pp_commit_row(long long *rows, int i, int W, P p) {
+    long long *row = rows + (long long)i * W;
+    long long paired = 0;
+    for (int k = 0; k < i - TURN; k++) paired += llrint(p(k, i) * PP_UNIT);
+    for (int l = i + TURN + 1; l < W; l++) {
+        const long long v = llrint(p(i, l) * PP_UNIT);
+        if (v) atomicAdd(reinterpret_cast<unsigned long long *>(row + (l - i)), (unsigned long long)v);
+        paired += v;
+    }
+    if (paired) atomicAdd(reinterpret_cast<unsigned long long *>(row), (unsigned long long)paired);
+}
+
+// rows [row0, row0 + n_rows) of D += src (same layout)
+void launch_pairprob_merge(const PairProbDense &D, int row0, int n_rows, const long long *src, cudaStream_t stream,
+                           int *n_launches);
+// rows [row0, row0 + n_rows): paired[r] = column 0 / n(i); npairs[r] = pairs (i, j) with P(i, j) >= cutoff;
+// offsets[n_rows + 1] = their exclusive scan
+void launch_pairprob_count(const PairProbDense &D, int row0, int n_rows, double cutoff, double *paired, int32_t *npairs,
+                           long long *offsets, cudaStream_t stream, int *n_launches);
+// the pairs counted above, row then column order: 1-based i, j and P(i, j)
+void launch_pairprob_emit(const PairProbDense &D, int row0, int n_rows, double cutoff, const long long *offsets,
+                          int32_t *pi, int32_t *pj, double *prob, cudaStream_t stream, int *n_launches);
 
 }  // namespace sfb

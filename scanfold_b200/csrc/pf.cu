@@ -136,8 +136,11 @@ __device__ __forceinline__ double group_sum(double v, int G) {
 #ifndef SFB_PF_MINB
 #define SFB_PF_MINB 6   // resident CTAs per SM: measured 3 -> 9.99 k, 4 -> 10.6 k, 6 -> 13.0 k, 8 -> 8.9 k windows/s at 200 nt
 #endif
+// PAIRPROB: the launch carries a pair-probability table; a fold whose dG and ED are finite commits p = P * qb of every cell
+// (both triangles are still in the CTA's scratch at its end)
+template <bool PAIRPROB>
 __global__ void __launch_bounds__(NT, SFB_PF_MINB) pf_kernel(PfLaunch L, const MfeTables *__restrict__ MT,
-                                                const PfTables *__restrict__ T) {
+                                                const PfTables *__restrict__ T, PairProbCommit pp) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int W = L.W;
     const int tid = threadIdx.x, lane = tid & 31;
@@ -603,6 +606,16 @@ __global__ void __launch_bounds__(NT, SFB_PF_MINB) pf_kernel(PfLaunch L, const M
             if (L.n_out_of_range && !(isfinite(dG) && isfinite(2. * s))) atomicAdd(L.n_out_of_range, 1);
         }
         for (int k = tid; k < W; k += NT) L.centroid[(long long)fold * W + k] = cen[k];
+        if constexpr (PAIRPROB) {
+            double s = 0.;   // as thread 0 formed it
+            for (int w = 0; w < NT / 32; w++) s += red[w];
+            const double dG = (-log(Z) - W * log(st->pf_scale)) * st->kT / 1000.;
+            if (isfinite(dG) && isfinite(2. * s)) {
+                long long *rows = pp.table + (pp.row0 + (long long)fold * pp.step) * W;
+                for (int i = tid; i < W; i += NT)
+                    pp_commit_row(rows, i, W, [&](int k, int l) { return Pm[TRI(l - k, k)] * qb[TRI(l - k, k)]; });
+            }
+        }
         __syncthreads();
     }
 #undef TRI
@@ -620,8 +633,8 @@ size_t pf_smem_bytes(int W) {
 
 }  // namespace
 
-size_t pf_scratch_doubles_per_cta(int W) {
-    const size_t a = 2 * ((size_t)W * (W + 1) / 2) + 6 * (size_t)W * W + 3 * (size_t)PRING * W, b = pf2_scratch_doubles_per_cta();
+size_t pf_scratch_doubles_per_cta(int W, bool pairprob) {
+    const size_t a = 2 * ((size_t)W * (W + 1) / 2) + 6 * (size_t)W * W + 3 * (size_t)PRING * W, b = pf2_scratch_doubles_per_cta(pairprob);
     return a > b ? a : b;
 }
 
@@ -637,20 +650,24 @@ int pf_grid_size(int W, int n_sm, int n_fold) {
 }
 
 void launch_pf(const PfLaunch &L, const MfeTables *d_mfe, const PfTables *d_pf, int n_sm, cudaStream_t stream,
-               int *n_launches) {
+               int *n_launches, const PairProbCommit &pp) {
     if (L.n_fold <= 0) return;
     if (pf2_supports(L)) {   // unconstrained windows up to 120 nt: shared-memory kernel (pf2.cu)
-        launch_pf2(L, d_mfe, d_pf, n_sm, stream, n_launches);
+        launch_pf2(L, d_mfe, d_pf, n_sm, stream, n_launches, pp);
         return;
     }
     size_t smem = pf_smem_bytes(L.W);
     static bool configured = false;
     if (!configured) {
-        cudaFuncSetAttribute(pf_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(227 * 1024));
+        cudaFuncSetAttribute(pf_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(227 * 1024));
+        cudaFuncSetAttribute(pf_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(227 * 1024));
         configured = true;
     }
     int grid = pf_grid_size(L.W, n_sm, L.n_fold);
-    pf_kernel<<<grid, NT, smem, stream>>>(L, d_mfe, d_pf);
+    if (pp.table)
+        pf_kernel<true><<<grid, NT, smem, stream>>>(L, d_mfe, d_pf, pp);
+    else
+        pf_kernel<false><<<grid, NT, smem, stream>>>(L, d_mfe, d_pf, pp);
     if (n_launches) (*n_launches)++;
 }
 

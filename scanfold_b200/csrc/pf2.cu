@@ -226,8 +226,11 @@ __device__ __forceinline__ double shape_out(const Smem2 &sm, const PfTables *T, 
 #define PF2_RESET
 #endif
 
+// PAIRPROB: the launch carries a pair-probability table; the outside pass stages every probability in the CTA's scratch
+// (L2 resident) and the fold commits them at its end, when its dG and ED are known to be finite
+template <bool PAIRPROB>
 __global__ void __launch_bounds__(NT2, 1)
-pf2_kernel(PfLaunch L, const MfeTables *__restrict__ MT, const PfTables *__restrict__ T) {
+pf2_kernel(PfLaunch L, const MfeTables *__restrict__ MT, const PfTables *__restrict__ T, PairProbCommit pp) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     Smem2 &sm = *reinterpret_cast<Smem2 *>(smem_raw);
     const int W = L.W;
@@ -235,6 +238,7 @@ pf2_kernel(PfLaunch L, const MfeTables *__restrict__ MT, const PfTables *__restr
     const unsigned full = 0xffffffffu;
     double *qbG = L.gscratch + (long long)blockIdx.x * L.gscratch_per_cta;   // qb[j][i], pitch P2
     double *pmG = qbG + P2 * P2;                                              // PM[j][i]
+    double *ppG = pmG + P2 * P2;                                              // PAIRPROB: p[l][k]
     const int HF = (W + 3) / 2;
     auto qmrow = [&](int kk) { return kk <= HF ? kk * PQ : (W + 3 - kk) * PQ + (W - kk); };   // + i
 #ifdef SFB_PF2_TIMING
@@ -743,7 +747,7 @@ pf2_kernel(PfLaunch L, const MfeTables *__restrict__ MT, const PfTables *__restr
             // ---- phase 2: P of the column, ring copies, PM, probabilities; X2 and qb of the next column
             if (tid < PP) {
                 const int k = tid;
-                double Pv = 0., vG = 0., v1 = 0., vB = 0., pm = 0.;
+                double Pv = 0., vG = 0., v1 = 0., vB = 0., pm = 0., pk = 0.;
                 if (k <= l - TURN - 1) {
                     const double qkl = sm.qcol[k];
                     if (qkl != 0.) {
@@ -765,6 +769,7 @@ pf2_kernel(PfLaunch L, const MfeTables *__restrict__ MT, const PfTables *__restr
                         }
                         pm = Pv * closing * TH->mlstem[rtype_of(t)][S[l - 1]][S[k + 1]];
                         const double p = Pv * qkl;
+                        pk = p;
                         ed_local += p * (1. - p);
                         if (p > 0.5) {
                             sm.cen[k] = (short)(l + 1);
@@ -773,6 +778,7 @@ pf2_kernel(PfLaunch L, const MfeTables *__restrict__ MT, const PfTables *__restr
                         if (L.bpp) L.bpp[((long long)fold * W + k) * W + l] = p;
                     }
                     pmG[l * P2 + k] = pm;
+                    if constexpr (PAIRPROB) ppG[l * P2 + k] = pk;
                 }
                 if (k < P2) {
                     const int o = (k + RPAD) * PT + (l & 31);
@@ -833,6 +839,15 @@ pf2_kernel(PfLaunch L, const MfeTables *__restrict__ MT, const PfTables *__restr
             if (L.n_out_of_range && !(isfinite(dG) && isfinite(2. * s))) atomicAdd(L.n_out_of_range, 1);
         }
         for (int k = tid; k < W; k += NT2) L.centroid[(long long)fold * W + k] = sm.cen[k];
+        if constexpr (PAIRPROB) {
+            // every thread forms the sum and dG as thread 0 did: commit only what the fold's outputs say is in range
+            double s = 0.;
+            for (int w = 0; w < NW2; w++) s += sm.red[w];
+            const double dG = (-log(Z) - W * log(T->pf_scale)) * T->kT / 1000.;
+            if (isfinite(dG) && isfinite(2. * s) && tid < W)
+                pp_commit_row(pp.table + (pp.row0 + (long long)fold * pp.step) * W, tid, W,
+                              [&](int k, int l) { return ppG[l * P2 + k]; });
+        }
 #ifdef SFB_PF2_TIMING
         if (blockIdx.x == 0 && fold == 0 && lane == 0)
             printf("pf2 timing warp %2d: inside p1 %lld wait %lld p2 %lld wait %lld | outside p1 %lld wait %lld p2 %lld wait %lld\n", warp,
@@ -856,7 +871,7 @@ bool pf2_supports(const PfLaunch &L) {
            L.W <= P2;   // the scale is baked into g_K2 and the shared scale row: a rescaled retry runs on pf.cu
 }
 
-size_t pf2_scratch_doubles_per_cta() { return 2 * (size_t)P2 * P2; }
+size_t pf2_scratch_doubles_per_cta(bool pairprob) { return (pairprob ? 3 : 2) * (size_t)P2 * P2; }
 
 void pf2_upload_tables(const PfTables &q) {
     static double kk[32 * 32];
@@ -882,15 +897,19 @@ void pf2_upload_tables(const PfTables &q) {
 }
 
 void launch_pf2(const PfLaunch &L, const MfeTables *d_mfe, const PfTables *d_pf, int n_sm, cudaStream_t stream,
-                int *n_launches) {
+                int *n_launches, const PairProbCommit &pp) {
     const size_t smem = sizeof(Smem2);
     static bool configured = false;
     if (!configured) {
-        cudaFuncSetAttribute(pf2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaFuncSetAttribute(pf2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaFuncSetAttribute(pf2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         configured = true;
     }
     const int grid = L.n_fold < n_sm ? L.n_fold : n_sm;
-    pf2_kernel<<<grid, NT2, smem, stream>>>(L, d_mfe, d_pf);
+    if (pp.table)
+        pf2_kernel<true><<<grid, NT2, smem, stream>>>(L, d_mfe, d_pf, pp);
+    else
+        pf2_kernel<false><<<grid, NT2, smem, stream>>>(L, d_mfe, d_pf, pp);
     if (n_launches) (*n_launches)++;
 }
 

@@ -22,7 +22,9 @@ EXPORTS = ["sfb_version", "sfb_init", "sfb_shutdown", "sfb_last_error", "sfb_par
            "sfb_fold_long", "sfb_pf_batch", "sfb_deigan", "sfb_scan", "sfb_scan_plan_create", "sfb_scan_plan_keep_shuffles",
            "sfb_scan_plan_run", "sfb_scan_plan_fetch", "sfb_scan_plan_stage_ms", "sfb_scan_plan_destroy", "sfb_accumulate_begin",
            "sfb_accumulate_geometry", "sfb_accumulate_export", "sfb_accumulate_merge", "sfb_accumulate_compact",
-           "sfb_accumulate_fetch", "sfb_accumulate_launches", "sfb_accumulate_free", "sfb_microbench", "sfb_set_stream", "sfb_set_engines"]
+           "sfb_accumulate_fetch", "sfb_accumulate_launches", "sfb_accumulate_free", "sfb_microbench", "sfb_set_stream", "sfb_set_engines",
+           "sfb_pairprob_begin", "sfb_scan_plan_pairprob", "sfb_pairprob_export", "sfb_pairprob_merge", "sfb_pairprob_compact",
+           "sfb_pairprob_fetch", "sfb_pairprob_free"]
 
 
 class EngineError(RuntimeError):
@@ -93,6 +95,14 @@ def load_library():
         L.sfb_accumulate_launches.argtypes = [C.c_void_p]
         L.sfb_accumulate_free.argtypes = [C.c_void_p]
         L.sfb_accumulate_free.restype = None
+        L.sfb_pairprob_begin.argtypes = [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_void_p)]
+        L.sfb_scan_plan_pairprob.argtypes = [C.c_void_p, C.c_void_p]
+        L.sfb_pairprob_export.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p]
+        L.sfb_pairprob_merge.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p]
+        L.sfb_pairprob_compact.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_double, C.POINTER(C.c_int64)]
+        L.sfb_pairprob_fetch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.sfb_pairprob_free.argtypes = [C.c_void_p]
+        L.sfb_pairprob_free.restype = None
         L.sfb_shutdown.restype = None
         L.sfb_set_stream.argtypes = [C.c_void_p]
         L.sfb_set_engines.argtypes = [C.c_int, C.c_int]
@@ -246,7 +256,7 @@ class ScanPlan:
 
     def __init__(self, seq, W, step, r, shuffle_type="mono", seed=42, parity_shuffles=None, temperature=37.0,
                  max_span=0, hc=None, react=None, shape_m=0.8, shape_b=-0.2, first_window=0, n_windows=None,
-                 final_window=True, want_pf=True, keep_shuffles=False, background_temperature=None):
+                 final_window=True, want_pf=True, keep_shuffles=False, background_temperature=None, pairprob=None):
         ensure_init()
         self._lib = load_library()
         self._seq = np.frombuffer(seq.encode() if isinstance(seq, str) else bytes(seq), dtype=np.uint8).copy()
@@ -293,8 +303,15 @@ class ScanPlan:
         self._keep = keep_shuffles
         if keep_shuffles:
             self._lib.sfb_scan_plan_keep_shuffles(self._plan)
+        if pairprob is not None:
+            self.attach_pairprob(pairprob)
         self.ms_total = self.ms_mfe = 0.0
         self.n_launches = 0
+
+    def attach_pairprob(self, table):
+        """every later run() adds the pair probabilities of this plan's regular windows to `table` (a PairProbTable)"""
+        _check(self._lib.sfb_scan_plan_pairprob(self._plan, table._h))
+        self._pairprob = table      # the table must outlive the plan's runs
 
     def run(self):
         ms_t, ms_m, nl = C.c_float(), C.c_float(), C.c_int32()
@@ -417,6 +434,82 @@ class Accumulator:
     def close(self):
         if self._h:
             self._lib.sfb_accumulate_free(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+PAIR_CUTOFF = 0.01     # pairs listed by --pair_probs (RNAplfold's -c default is 0.01 too)
+
+
+def windows_holding(i, j, W, step, n_windows):
+    """number of regular windows w in [0, n_windows) with w*step <= i and j < w*step + W (0-based, i <= j; arrays work)"""
+    i, j = np.asarray(i, dtype=np.int64), np.asarray(j, dtype=np.int64)
+    lo = np.where(j - W + 1 <= 0, 0, (j - W + 1 + step - 1) // step)
+    hi = np.minimum(i // step, n_windows - 1)
+    return np.maximum(hi - lo + 1, 0)
+
+
+class PairProbTable:
+    """Device-resident window-averaged base-pair probabilities of one shard of windows (sfb_pairprob_*).
+
+    rows = nucleotides [nt0, nt0 + n_nt) touched by the shard, 0-based; W int64 columns of exact fixed-point sums
+    (column 0: paired, d >= 1: pair (i, i+d)).  Attach it to the scan (scan.scan_record(..., pairprob=table)), move halo
+    rows with export_tensors() / merge_tensors() (multigpu.exchange_halo), then reduce() the rows this shard owns."""
+
+    def __init__(self, L, W, step, first_window, n_windows):
+        ensure_init()
+        self._lib = load_library()
+        self._h = C.c_void_p()
+        _check(self._lib.sfb_pairprob_begin(int(L), int(W), int(step), int(first_window), int(n_windows), C.byref(self._h)))
+        self.L, self.W, self.step = L, W, step
+        self.nt0, self.n_nt = first_window * step, (n_windows - 1) * step + W
+
+    def export_rows(self, row0, n_rows, d_rows):
+        _check(self._lib.sfb_pairprob_export(self._h, row0, n_rows, d_rows))
+
+    def merge_rows(self, row0, n_rows, d_rows):
+        _check(self._lib.sfb_pairprob_merge(self._h, row0, n_rows, d_rows))
+
+    # ---- torch views of the halo rows (multi-GPU exchange over NCCL, scanfold_b200.multigpu)
+    def empty_tensors(self, n_rows):
+        import torch
+        return (torch.empty(n_rows * self.W, dtype=torch.int64, device="cuda"),)
+
+    def export_tensors(self, row0, n_rows):
+        t = self.empty_tensors(n_rows)
+        self.export_rows(row0, n_rows, t[0].data_ptr())
+        return t
+
+    def merge_tensors(self, row0, n_rows, rows):
+        self.merge_rows(row0, n_rows, rows.data_ptr())
+
+    def rows(self, row0=0, n_rows=None):
+        """the raw int64 sums of rows [row0, row0 + n_rows) as a numpy [n_rows, W] array (tests)"""
+        n_rows = self.n_nt - row0 if n_rows is None else n_rows
+        t = self.export_tensors(row0, n_rows)[0]
+        return t.cpu().numpy().reshape(n_rows, self.W)
+
+    def reduce(self, row0=0, n_rows=None, cutoff=PAIR_CUTOFF):
+        """-> (paired [n_rows] float64, i, j [M] int32 1-based, p [M] float64): the pairs with P >= cutoff, by i then j"""
+        if n_rows is None:
+            n_rows = self.n_nt - row0
+        m = C.c_int64()
+        _check(self._lib.sfb_pairprob_compact(self._h, row0, n_rows, float(cutoff), C.byref(m)))
+        M = m.value
+        paired = np.zeros(max(n_rows, 1))
+        i, j = np.zeros(max(M, 1), dtype=np.int32), np.zeros(max(M, 1), dtype=np.int32)
+        p = np.zeros(max(M, 1))
+        _check(self._lib.sfb_pairprob_fetch(self._h, paired.ctypes.data, i.ctypes.data, j.ctypes.data, p.ctypes.data))
+        return paired[:n_rows], i[:M], j[:M], p[:M]
+
+    def close(self):
+        if self._h:
+            self._lib.sfb_pairprob_free(self._h)
             self._h = C.c_void_p()
 
     def __del__(self):

@@ -155,6 +155,26 @@ def empty_table():
     return foldstep.PartnerTable(np.zeros(1, dtype=np.int64), z, z, z, np.zeros((6, 0), dtype=np.int64), z)
 
 
+def pairprob_distributed(table, W, step, rank, world, dist, total_windows, cutoff):
+    """Window-averaged pair probabilities of the whole record on rank 0: halo exchange of the PairProbTable rows (exact
+    integer sums, so any sharding gives the same result), every rank reduces the rows it owns, rank 0 gathers them.
+    `table` is None on a rank without windows.  -> (paired [nucleotides up to the end of the last window], i, j, p) on
+    rank 0, None elsewhere.  Nucleotides no window holds (step > W) belong to no rank and stay 0."""
+    own = exchange_halo(table, W, step, rank, world, dist, total_windows)
+    if table is not None and own > 0:
+        part = list(table.reduce(0, own, cutoff))
+    else:
+        part = [np.zeros(0), np.zeros(0, dtype=np.int32), np.zeros(0, dtype=np.int32), np.zeros(0)]
+    parts = gather_arrays(part, rank, world, dist)
+    if rank != 0:
+        return None
+    rows = shard_rows(total_windows, world, W, step)
+    paired = np.zeros(max(r[1] for r in rows))
+    for r, p in zip(rows, parts):
+        paired[r[2]:r[2] + len(p[0])] = p[0]
+    return (paired,) + tuple(np.concatenate([p[k] for p in parts]) for k in range(1, 4))
+
+
 def own_partner_table(acc, W, step, rank, world, dist, total_windows):
     """halo exchange + compaction: the complete partner lists of the nucleotides this rank owns"""
     own = exchange_halo(acc, W, step, rank, world, dist, total_windows)

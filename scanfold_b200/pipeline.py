@@ -46,6 +46,18 @@ class RunNames:
         self.dbn1, self.dbn2, self.dbn3, self.dbn4 = dbn1, dbn2, dbn3, dbn4
 
 
+def write_pairprob_outputs(pairprob, names, W, step, total_windows):
+    """the three files of --pair_probs: paired(i) track, pair list (P >= 0.01), IGV arcs (P >= 0.1)"""
+    from . import engine
+    paired, i, j, p = pairprob
+    pos = np.arange(len(paired))
+    covered = engine.windows_holding(pos, pos, W, step, total_windows) > 0
+    o = names.outname
+    writers.write_pairprob_wig(o + ".pairprob.wig", paired, covered, names.name)
+    writers.write_pairprob_txt(o + ".pairprob.txt", i, j, p)
+    writers.write_pairprob_bp(names.out6 + "." + o + ".pairprob.bp", i, j, p, names.name)
+
+
 def zscore_total(table):
     """the reference's zscore_total (ScanFold.py:556,751): every numeric z of the scan loop plus the final-window one"""
     alln = table.alln if getattr(table, "alln", None) is not None else np.zeros(len(table), dtype=bool)

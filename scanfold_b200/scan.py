@@ -114,12 +114,14 @@ def table_from_result(res, first_window, step, n_regular, final_window):
 
 def scan_record(seq, W=120, step=1, r=100, shuffle_type="mono", seed=42, parity_shuffles=None, temperature=37.0,
                 max_span=0, hc=None, react=None, shape_m=0.8, shape_b=-0.2, first_window=0, n_windows=None,
-                final_window=None, want_pf=True, background_temperature=None):
+                final_window=None, want_pf=True, background_temperature=None, pairprob=None):
     """Scan one record (or the window range [first_window, first_window + n_windows) of it).
 
     seq: RNA string (T already transcribed, ScanFold.py:282).  hc: line 3 of --constraints (one char per
     nt) or None.  react: 1-based reactivity list (index 0 unused, -999 = missing) or None.
     final_window: evaluate the extra final-window set; default = this shard holds the last window.
+    pairprob: an engine.PairProbTable whose range holds these windows; every part of the scan adds its windows' pair
+    probabilities to it.
     """
     L = len(seq)
     total = n_windows_of(L, W, step)
@@ -130,7 +132,8 @@ def scan_record(seq, W=120, step=1, r=100, shuffle_type="mono", seed=42, parity_
     if final_window is None:
         final_window = first_window + n_windows == total
     kw = dict(shuffle_type=shuffle_type, seed=seed, temperature=temperature, max_span=max_span, hc=hc, react=react,
-              shape_m=shape_m, shape_b=shape_b, want_pf=want_pf, background_temperature=background_temperature)
+              shape_m=shape_m, shape_b=shape_b, want_pf=want_pf, background_temperature=background_temperature,
+              pairprob=pairprob)
     if n_windows <= PIPELINE_WINDOWS:
         res = engine.scan(seq, W, step, r, parity_shuffles=parity_shuffles, first_window=first_window,
                           n_windows=n_windows, final_window=final_window, **kw)

@@ -3,6 +3,7 @@
   makedbn              ScanFoldFunctions.py:67-138  write_bp       :644-712
   write_wig            :626-642                     write_wig_dict :616-624
   write_fasta          :597-605
+and the additive pair-probability files of --pair_probs (write_pairprob_*), which have no reference counterpart.
 The reference's CT files can be asymmetric (i -> j while j -> 0, Appendix B Q14); makedbn's '<' / '>'
 symbols for non-nested partners are reproduced from the CT rows, not from a pair table.
 """
@@ -174,6 +175,38 @@ def write_wig_dict(path, z_arr, name, step):
     with open(path, "w") as f:
         f.write("fixedStep chrom=%s start=1 step=%s span=%s\n" % (name, step, step))
         f.write("".join("%f\n" % v for v in z_arr.tolist()))
+
+
+def write_pairprob_wig(path, paired, covered, name):
+    """paired(i) per nucleotide as a variableStep track; nucleotides no window holds (covered False) are left out"""
+    pos = np.nonzero(covered)[0]
+    with open(path, "w") as f:
+        f.write("variableStep chrom=%s span=1\n" % name)
+        f.write("".join("%d\t%f\n" % (k + 1, v) for k, v in zip(pos.tolist(), np.asarray(paired)[pos].tolist())))
+
+
+def write_pairprob_txt(path, i_arr, j_arr, p_arr):
+    """the listed pairs, 1-based, sorted by i then j"""
+    with open(path, "w") as f:
+        f.write("i\tj\tprobability\n")
+        f.write("".join("%d\t%d\t%.6f\n" % r for r in zip(i_arr.tolist(), j_arr.tolist(), p_arr.tolist())))
+
+
+PAIRPROB_BP_CLASSES = ((0.1, "color:\t199\t199\t199\t0.1 to 0.3\n"), (0.3, "color:\t236\t236\t136\t0.3 to 0.5\n"),
+                       (0.5, "color:\t89\t222\t111\t0.5 to 0.8\n"), (0.8, "color:\t55\t129\t255\t0.8 to 1\n"))
+
+
+def write_pairprob_bp(path, i_arr, j_arr, p_arr, name):
+    """IGV arc track in the layout of write_bp: the pairs with P >= 0.1, colour class = the last column"""
+    lows = np.array([c[0] for c in PAIRPROB_BP_CLASSES])
+    p_arr = np.asarray(p_arr)
+    keep = p_arr >= lows[0]
+    cls = np.searchsorted(lows, p_arr[keep], side="right") - 1
+    rows = [c[1] for c in PAIRPROB_BP_CLASSES]
+    rows += ["%s\t%d\t%d\t%d\t%d\t%d\n" % (name, i, i, j, j, c)
+             for i, j, c in zip(np.asarray(i_arr)[keep].tolist(), np.asarray(j_arr)[keep].tolist(), cls.tolist())]
+    with open(path, "w") as f:
+        f.write("".join(rows))
 
 
 def write_fasta(path, seq, name):
