@@ -148,7 +148,8 @@ __global__ void __launch_bounds__(NT, SFB_PF_MINB) pf_kernel(PfLaunch L, const M
 
     PfSmall *st = reinterpret_cast<PfSmall *>(smem_raw);
     double *dp = reinterpret_cast<double *>(smem_raw + ((sizeof(PfSmall) + 15) & ~15));
-    double *scale = dp;   dp += W + 4;
+    const int nscale = max(W, MAXLOOP) + 4;   // st->fac reads scale[u1 + u2 + 2] up to MAXLOOP + 2 at every W
+    double *scale = dp;   dp += nscale;
     double *eMLb = dp;    dp += W + 4;
     double *q5 = dp;      dp += W + 2;
     double *q3 = dp;      dp += W + 2;
@@ -219,10 +220,8 @@ __global__ void __launch_bounds__(NT, SFB_PF_MINB) pf_kernel(PfLaunch L, const M
             }
             scale[0] = 1.;
             eMLb[0] = 1.;
-            for (int k = 1; k < W + 4; k++) {
-                scale[k] = scale[k - 1] / st->pf_scale;
-                eMLb[k] = eMLb[k - 1] * T->expMLbase / st->pf_scale;
-            }
+            for (int k = 1; k < nscale; k++) scale[k] = scale[k - 1] / st->pf_scale;
+            for (int k = 1; k < W + 4; k++) eMLb[k] = eMLb[k - 1] * T->expMLbase / st->pf_scale;
         }
     }
     __syncthreads();
@@ -625,7 +624,7 @@ __global__ void __launch_bounds__(NT, SFB_PF_MINB) pf_kernel(PfLaunch L, const M
 
 size_t pf_smem_bytes(int W) {
     size_t b = (sizeof(PfSmall) + 15) & ~(size_t)15;
-    b += sizeof(double) * (2 * (W + 4) + 2 * (W + 2) + 8);
+    b += sizeof(double) * ((std::max(W, MAXLOOP) + 4) + (W + 4) + 2 * (W + 2) + 8);
     b += sizeof(int) * ((W + 2) + 4 + (W + 2));
     b += sizeof(int16_t) * 3 * W + 3 * (W + 4);
     return (b + 15) & ~(size_t)15;
